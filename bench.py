@@ -10,6 +10,12 @@ regulariser) for a fixed parameter vector.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--scaling weak|strong]
                     [--precision fp32|bf16] [--seqs N --sites L] [--workload plm|hamming|fit]
+                    [--dump-outputs DIR]
+
+--dump-outputs DIR: after the timed steps, write what the timed path computed in its last step as DIR/<name>.npy
+(float32 / float64): for `plm` the gradient (`gradient`) and [-loglk, objective] (`fx`), for `hamming` the
+neighbour counts (`counts`).  Inputs are seeded, so two builds run with the same arguments can be compared
+output for output.
 
 N > 1: launched by torchrun, one rank per GPU; sequences sharded over ranks, ONE NCCL all-reduce of
 [gradient, -loglk] (n + 4 floats) per step.  Default `weak`: 50,000 sequences per GPU (the 8-GPU point is the
@@ -46,6 +52,8 @@ METRIC = "PLM gradient evals/s as N*L^2*q cell-ops/s"
 UNIT = "cell-ops/s"
 ACC_SAMPLE_N = 5000
 CPU_BUDGET_S = 150.0
+DUMP_LIMIT_BYTES = 64 << 20
+DUMP_SEED = 0
 
 
 def host_threads():
@@ -148,6 +156,29 @@ def make_inputs(n_total):
     n = L * Q + L * (L - 1) // 2 * Q * Q
     x = np.random.default_rng(SEED).normal(0.0, 0.05, n).astype(np.float32)
     return codes, x
+
+
+def dump_outputs(directory, arrays):
+    """Writes each array as DIR/<name>.npy.  An array too large for the DUMP_LIMIT_BYTES budget left by the others
+    is replaced by a fixed, seeded sample of its elements (<name>.npy) and their flat positions (<name>_index.npy,
+    float64).  Returns the names written."""
+    os.makedirs(directory, exist_ok=True)
+    budget = DUMP_LIMIT_BYTES
+    written = []
+    for name, a in sorted(arrays.items(), key=lambda kv: kv[1].nbytes):
+        a = np.ascontiguousarray(a)
+        if a.nbytes > budget:
+            a = a.reshape(-1)
+            k = budget // (a.itemsize + 8)
+            idx = np.unique(np.random.default_rng(DUMP_SEED).integers(0, a.size, k))
+            np.save(os.path.join(directory, name + "_index.npy"), idx.astype(np.float64))
+            written.append(name + "_index")
+            budget -= idx.size * 8
+            a = a[idx]
+        np.save(os.path.join(directory, name + ".npy"), a)
+        written.append(name)
+        budget -= a.nbytes
+    return written
 
 
 def cpu_arm(codes, x, weights, steps, warmup, budget_s=CPU_BUDGET_S):
@@ -336,6 +367,9 @@ def run_b200(args):
     ev1.record()
     barrier()
     ms_total = ev0.elapsed_time(ev1)
+    if args.dump_outputs and rank == 0:
+        # the last timed step's results, before anything else reuses the buffers
+        outputs = {"gradient": prob.g.cpu().numpy(), "fx": prob.fxbuf.cpu().numpy()}
     launches = engine.kernel_launches - launches0
     t = torch.tensor([ms_total], dtype=torch.float64, device=engine.device)
     if world > 1:
@@ -537,6 +571,8 @@ def run_b200(args):
             line["hamming"]["unpruned"] = hamming_unpruned_ms()
         except Exception as e:
             line["hamming"] = {"error": "%s: %s" % (type(e).__name__, e)}
+    if args.dump_outputs and rank == 0:
+        line["dumped_outputs"] = dump_outputs(args.dump_outputs, outputs)
     if world > 1:
         dist.destroy_process_group()
     _nccl_log_to_stderr(nccl_dir)
@@ -714,6 +750,8 @@ def run_hamming(args):
         line["cpu_baseline"] = {"value": rows * N / dt / 2, "unit": "pairs/s", "cores": host_threads(), "kind": "port",
                                 "sample": "%d of %d rows against all columns (%.1f s); unordered-pair equivalent" % (rows, N, dt)}
         line["parity_sample_rows_exact"] = bool(np.array_equal(got[:rows], ref))
+    if args.dump_outputs and rank == 0:
+        line["dumped_outputs"] = dump_outputs(args.dump_outputs, {"counts": d_counts.cpu().numpy().astype(np.float64)})
     if world > 1:
         dist.destroy_process_group()
     _nccl_log_to_stderr(nccl_dir)
@@ -740,7 +778,13 @@ def main():
     ap.add_argument("--backward", default=None, choices=["gather", "tc"],
                     help="backward kernel of the data term (default: engine default / EVC_BACKWARD)")
     ap.add_argument("--no-subrecords", action="store_true", help="skip the hamming / fit / run_plmc sub-records")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs as DIR/<name>.npy (at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     global N_PER_GPU, L, LAMBDA_J
     if args.seqs:
         N_PER_GPU = args.seqs

@@ -627,10 +627,11 @@ def test_intree_twin_dropins_vs_reference_outputs(engine, golden_dir):
         assert np.allclose(fij[3, 3][np.arange(21), np.arange(21)], fi[3])
 
 
-def test_identities_to_seq_and_set_weights_vs_reference_class(engine):
-    """f3: identities_to_seq (alignment.py:1156-1189) and Alignment.set_weights (:899-930) drop-ins.  When the
-    reference is importable (baseline/_ref on the GPU box) the reference's own numba function and Alignment class
-    are the comparison; the definition (row-wise equality count) always is."""
+def test_identities_to_seq_and_set_weights_vs_reference_class(engine, golden_dir):
+    """f3: identities_to_seq (alignment.py:1156-1189) and Alignment.set_weights (:899-930) drop-ins.  The
+    reference's own numba function and Alignment class are the comparison (their outputs on a seeded alignment
+    stored by tests/golden/make_golden.py); the definition (row-wise equality count) always is."""
+    import types
     from evcouplings_b200 import alignment as ga
     rng = np.random.default_rng(5)
     for N, L in ((1, 1), (257, 33), (5000, 301)):
@@ -640,24 +641,20 @@ def test_identities_to_seq_and_set_weights_vs_reference_class(engine):
         assert got.dtype == np.float64 and np.array_equal(got, (m == s[None, :]).sum(axis=1).astype(np.float64))
     with pytest.raises(ValueError):
         ga.frequencies(np.full((4, 3), 21), np.ones(4), 21, engine=engine)        # symbol out of range
-    import ref_harness
-    if not ref_harness.available():
-        return
-    ref_harness.install()
-    from evcouplings.align.alignment import Alignment, identities_to_seq as ref_ids
-    codes = synthetic.synthetic_msa_codes(300, 25, 9)
-    seqs = ["".join(synthetic.ALPHABET[c] for c in row) for row in codes]
-    ali_ref = Alignment.from_dict({"s%d" % k: v for k, v in enumerate(seqs)})
-    ali_gpu = Alignment.from_dict({"s%d" % k: v for k, v in enumerate(seqs)})
-    f_before = ali_gpu.frequencies.copy()                  # cached, unweighted
-    ali_ref.set_weights(0.8)
-    ga.set_weights(ali_gpu, 0.8, engine=engine)
-    assert np.array_equal(ali_gpu.num_cluster_members, ali_ref.num_cluster_members)
-    assert np.array_equal(ali_gpu.weights, ali_ref.weights)
+    d = np.load(os.path.join(golden_dir, "reference_boundary.npz"))
+    mapped = d["ali_matrix_mapped"].astype(np.int64)
+    # the reference's Alignment.matrix_mapped of synthetic_msa_codes(300, 25, 9) is those codes
+    assert np.array_equal(mapped, synthetic.synthetic_msa_codes(300, 25, 9).astype(np.int64))
+    ali = types.SimpleNamespace(matrix_mapped=mapped, _frequencies=d["ali_frequencies_unweighted"],
+                                _pair_frequencies=None)
+    ga.set_weights(ali, 0.8, engine=engine)
+    assert np.array_equal(ali.num_cluster_members, d["ali_num_cluster_members"])
+    assert np.array_equal(ali.weights, d["ali_weights"])
     # the drop-in resets the cached frequencies like the reference does: the next access is weighted
-    assert np.allclose(ali_gpu.frequencies, ali_ref.frequencies) and not np.allclose(ali_gpu.frequencies, f_before)
-    mapped = ali_ref.matrix_mapped
-    assert np.array_equal(ga.identities_to_seq(mapped[0], mapped, engine=engine), ref_ids(mapped[0], mapped))
+    assert ali._frequencies is None and ali._pair_frequencies is None
+    fw = ga.frequencies(mapped, ali.weights, 21, engine=engine)
+    assert np.allclose(fw, d["ali_frequencies"]) and not np.allclose(fw, d["ali_frequencies_unweighted"])
+    assert np.array_equal(ga.identities_to_seq(mapped[0], mapped, engine=engine), d["ali_identities_to_first"])
 
 
 # ------------------------------------------------------------------------------------------------

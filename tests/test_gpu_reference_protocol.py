@@ -1,35 +1,30 @@
 """
-Drop-in boundary on the GPU (-m gpu): the reference's OWN couplings protocol and its OWN run_plmc run unmodified
-over the CUDA engine.  The reference is imported from the git-ignored install baseline/_ref
-(scripts/install_reference.sh), which travels to the GPU box; /root/reference is never read there.
+Drop-in boundary on the GPU (-m gpu): the calls the reference's OWN couplings protocol and its OWN run_plmc make
+into our boundary, recorded with the unmodified reference (tests/golden/make_golden.py, reference_boundary),
+are replayed over the CUDA engine, and what we return and write is checked against what the reference's stage
+code and readers made of it (see tests/reference_golden.py).
 
   1. primary plug point: evcouplings.couplings.protocol.run(protocol="standard") (protocol.py:363-429 ->
-     infer_plmc :56-257) with ct.run_plmc = evcouplings_b200.run_plmc (CudaEngine, default tcgen05 path);
-  2. secondary plug point: the reference's run_plmc (tools.py:126-307: argv, subprocess, stderr parsing, file
-     checks) drives bin/evcplm-plmc, i.e. the real executable with the real engine.
+     infer_plmc :56-257) calling evcouplings_b200.run_plmc (CudaEngine, default tcgen05 path);
+  2. secondary plug point: the argv the reference's run_plmc (tools.py:126-307) builds drives bin/evcplm-plmc,
+     i.e. the real executable with the real engine, and its stderr is parsed as the reference parses it.
 """
 import os
+import subprocess
 
 import numpy as np
 import pytest
 
-import ref_harness
+import reference_golden as rg
 
-pytestmark = [pytest.mark.gpu,
-              pytest.mark.skipif(not ref_harness.available(),
-                                 reason="reference not installed (run scripts/install_reference.sh)")]
+pytestmark = pytest.mark.gpu
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 @pytest.fixture(scope="module")
 def ref():
-    ref_harness.install()
-    import evcouplings.couplings.tools as ct
-    import evcouplings.couplings.protocol as cpr
-    import evcouplings.couplings.model as cm
-    import evcouplings.couplings.pairs as cp
-    return dict(ct=ct, cpr=cpr, cm=cm, cp=cp)
+    return rg.load()
 
 
 @pytest.fixture(scope="module")
@@ -38,64 +33,36 @@ def engine():
     return CudaEngine()
 
 
-def _kwargs(prefix, a2m, L, ignore_gaps, iterations):
-    return dict(
-        protocol="standard", prefix=prefix, alignment_file=a2m, focus_mode=True, focus_sequence="seq0/1-%d" % L,
-        theta=0.8, alphabet=None, segments=[["A_1", "aa", "seq0", 1, L, list(range(1, L + 1))]],
-        ignore_gaps=ignore_gaps, iterations=iterations, lambda_h=0.01, lambda_J=0.01, lambda_J_times_Lq=True,
-        lambda_group=None, scale_clusters=None, cpu=1, plmc="plmc", reuse_ecs=False, min_sequence_distance=6,
-        frequencies_file=None, scoring_model="skewnormal",
-    )
-
-
 @pytest.mark.parametrize("ignore_gaps", [True, False])
 def test_reference_standard_protocol_over_cuda_engine(ref, engine, tmp_path, ignore_gaps):
-    """BASELINE configs[0] (N=200, L=40) through the reference's stage driver, numerics on the B200."""
+    """BASELINE configs[0] (N=200, L=40) through the reference's stage driver's call, numerics on the B200."""
     from evcouplings_b200 import synthetic, tools
     from cpu_engine import OracleEngine
     from oracle import plm_oracle as po
+    meta, arr = ref
+    name = "standard_it40_ig%d" % int(ignore_gaps)
+    rec = meta[name]
     N, L = 200, 40
     codes = synthetic.synthetic_msa_codes(N, L, 1)
     a2m = str(tmp_path / "cfg1.a2m")
     synthetic.write_a2m(a2m, codes)
-    captured = {}
-
-    def run_plmc(*args, **kwargs):
-        res, run = tools.run_plmc(*args, engine=engine, return_run=True, num_gpus=1, **kwargs)
-        captured["run"], captured["kwargs"] = run, kwargs
-        return res
-
-    ct = ref["ct"]
-    original = ct.run_plmc
-    ct.run_plmc = run_plmc
-    try:
-        prefix = str(tmp_path / "out" / "job")
-        outcfg = ref["cpr"].run(**_kwargs(prefix, a2m, L, ignore_gaps, 40))
-    finally:
-        ct.run_plmc = original
+    args = [rg.subst(a, tmp_path) for a in rec["args"]]
+    kwargs = {k: rg.subst(v, tmp_path) for k, v in rec["kwargs"].items()}
     q_eff = 20 if ignore_gaps else 21
     lam_J = 0.01 * (q_eff - 1) * (L - 1)
-    assert abs(captured["kwargs"]["lambda_J"] - lam_J) < 1e-12           # protocol.py:157-179
-    for key in ("model_file", "raw_ec_file", "ec_file"):
-        assert os.path.getsize(outcfg[key]) > 0
-    assert outcfg["num_sites"] == L and outcfg["num_valid_sequences"] == N and outcfg["region_start"] == 1
-    run = captured["run"]
-    assert abs(outcfg["effective_sequences"] - run.n_eff) < 0.06
+    assert abs(kwargs["lambda_J"] - lam_J) < 1e-12           # protocol.py:157-179
+    assert kwargs["iterations"] == 40
+    res, run = tools.run_plmc(*args, engine=engine, return_run=True, num_gpus=1, **kwargs)
+    rg.check_result_as_protocol_reads_it(meta, rec, res, run)
+    assert rec["outcfg"]["num_sites"] == L and rec["outcfg"]["num_valid_sequences"] == N
     # the reference's readers on the files the CUDA engine wrote
-    model = ref["cm"].CouplingsModel(outcfg["model_file"])
-    assert model.L == L and model.num_symbols == q_eff and model.N_valid == N
-    h = run.x[:L * q_eff].reshape(L, q_eff)
-    assert np.array_equal(model.h_i, h.astype(np.float64))
-    iu, ju = np.triu_indices(L, 1)
-    J = run.x[L * q_eff:].reshape(-1, q_eff, q_eff)
-    assert np.array_equal(model.J_ij[iu, ju], J.astype(np.float64))
-    ecs = ref["cp"].read_raw_ec_file(outcfg["raw_ec_file"], sort=False)
-    assert len(ecs) == L * (L - 1) // 2
-    assert np.abs(ecs["cn"].values - po.cn_scores(J.astype(np.float64), L)).max() < 2e-6
-    it_ref, fields_ref = ct.parse_plmc_log(run.log)
-    it_own, fields_own = tools.parse_plmc_log(run.log)
-    assert fields_ref == fields_own and it_ref.equals(it_own) and len(it_ref) == 40
-    assert fields_ref[-1] == "LBFGSERR_MAXIMUMITERATION"
+    m = rg.check_model_as_reference_reads_it(rec, res.param_file, run)
+    assert m["L"] == L and m["q"] == q_eff and m["n_valid"] == N
+    J = m["J"].astype(np.float64)
+    ecs = rg.check_ecs_as_reference_reads_them(arr, name, res.couplings_file, J, L)
+    assert np.abs(ecs["cn"] - po.cn_scores(J, L)).max() < 2e-6
+    it_own = rg.check_log_as_reference_parses_it(rec, run.log, 40)
+    assert rec["log_fields"][-1] == "LBFGSERR_MAXIMUMITERATION"
     # same host logic over the float64 oracle backend from the same start, same iteration cap: the objective the
     # CUDA engine reached is the oracle's to fp32 noise (device L-BFGS = the same algorithm)
     r2, run2 = tools.run_plmc(a2m, str(tmp_path / "c_ECs.txt"), str(tmp_path / "c.model"), focus_seq="seq0/1-40",
@@ -105,33 +72,37 @@ def test_reference_standard_protocol_over_cuda_engine(ref, engine, tmp_path, ign
     f2 = r2.iteration_table["fx"].astype(float).values
     assert np.abs(f1 - f2).max() <= 2e-5 * np.abs(f2).max()
     cn2 = np.loadtxt(str(tmp_path / "c_ECs.txt"), usecols=5)
-    assert np.sqrt(np.mean((ecs["cn"].values - cn2) ** 2)) < 2e-3
+    assert np.sqrt(np.mean((ecs["cn"] - cn2) ** 2)) < 2e-3
+    # and so are the ECs the reference read from the oracle run when the fixture was recorded
+    assert np.sqrt(np.mean((ecs["cn"] - arr[name + "_ecs_cn"]) ** 2)) < 2e-3
 
 
 def test_unmodified_reference_run_plmc_over_real_executable(ref, tmp_path):
-    """The reference's run_plmc (subprocess + stderr scraping) over bin/evcplm-plmc with the CUDA engine."""
-    from evcouplings_b200 import synthetic
+    """The reference's run_plmc argv (subprocess + stderr scraping) over bin/evcplm-plmc with the CUDA engine."""
+    from evcouplings_b200 import synthetic, tools
     from oracle import plm_oracle as po
+    meta, _ = ref
+    rec = meta["cli_gpu"]
     codes = synthetic.synthetic_msa_codes(300, 24, 3)
-    a2m = str(tmp_path / "in.a2m")
-    synthetic.write_a2m(a2m, codes)
-    ecs, model = str(tmp_path / "o" / "x_ECs.txt"), str(tmp_path / "o" / "x.model")
-    env_before = os.environ.get("EVC_NUM_GPUS")
-    os.environ["EVC_NUM_GPUS"] = "1"
-    try:
-        res = ref["ct"].run_plmc(a2m, ecs, model, focus_seq="seq0/1-24", alphabet=None, theta=0.8, scale=None,
-                                 ignore_gaps=True, iterations=20, lambda_h=0.01, lambda_J=4.0, lambda_g=None, cpu=2,
-                                 binary=os.path.join(ROOT, "bin", "evcplm-plmc"))
-    finally:
-        if env_before is None:
-            os.environ.pop("EVC_NUM_GPUS", None)
-        else:
-            os.environ["EVC_NUM_GPUS"] = env_before
-    assert res.num_valid_seqs == 300 and res.num_total_seqs == 300 and res.num_valid_sites == 24
-    assert res.focus_seq_index == 1 and res.region_start == 1
-    assert res.optimization_status == "LBFGSERR_MAXIMUMITERATION" and len(res.iteration_table) == 20
+    synthetic.write_a2m(str(tmp_path / "in.a2m"), codes)
+    argv = [rg.subst(a, tmp_path) for a in rec["argv"]]
+    env = dict(os.environ, EVC_NUM_GPUS="1")
+    p = subprocess.run([os.path.join(ROOT, "bin", "evcplm-plmc")] + argv, capture_output=True, text=True, env=env)
+    assert p.returncode == 0, p.stderr
+    it, fields = tools.parse_plmc_log(p.stderr)
+    want = rec["result"]
+    ecs, model = rg.subst(want["couplings_file"], tmp_path), rg.subst(want["param_file"], tmp_path)
+    assert os.path.getsize(ecs) > 0 and os.path.getsize(model) > 0
+    got = dict(zip(["focus_seq_index", "num_valid_seqs", "num_total_seqs", "num_valid_sites", "num_total_sites",
+                    "region_start", "effective_samples", "optimization_status"], fields))
+    assert abs(got.pop("effective_samples") - want["effective_samples"]) < 0.06
+    assert got == {k: v for k, v in want.items() if k in got}
+    assert got["num_valid_seqs"] == 300 and got["num_total_seqs"] == 300 and got["num_valid_sites"] == 24
+    assert got["focus_seq_index"] == 1 and got["region_start"] == 1
+    assert got["optimization_status"] == "LBFGSERR_MAXIMUMITERATION"
+    assert list(it.columns) == rec["iter_columns"] and len(it) == rec["iter_len"] == 20
     m = po.read_model(model)
     assert (m["L"], m["q"], m["num_iter"]) == (24, 20, 20) and abs(m["lambda_J"] - 4.0) < 1e-6
-    assert abs(res.effective_samples - m["n_eff"]) < 0.06
-    fx = res.iteration_table["fx"].astype(float).values
+    assert abs(fields[6] - m["n_eff"]) < 0.06
+    fx = it["fx"].astype(float).values
     assert np.all(np.diff(fx) <= 1e-6 * np.abs(fx[:-1]))          # monotone descent

@@ -1,41 +1,27 @@
 """
-Drop-in boundary test (CPU, this container only): the reference's OWN couplings protocol
-(evcouplings/couplings/protocol.py:363-429 ``standard`` -> ``infer_plmc`` :56-257) runs unmodified with
-``evcouplings.couplings.tools.run_plmc`` replaced by ``evcouplings_b200.run_plmc``; the reference's own
-readers (CouplingsModel model.py:317-400, read_raw_ec_file pairs.py:34-65, parse_plmc_log tools.py:20-108)
-consume what we write.  The numerical engine injected here is the test-only oracle engine (no GPU in this
-container); the same host code runs over the CUDA engine in tests/test_gpu_parity.py.
-Skipped where /root/reference does not exist (the GPU box).
+Drop-in boundary test (CPU): the calls the reference's OWN couplings protocol
+(evcouplings/couplings/protocol.py:363-429 ``standard`` -> ``infer_plmc`` :56-257, and ``complex``) makes into
+``run_plmc``, and the argv its own ``run_plmc`` (tools.py:126-307) builds for a plmc executable, are replayed
+from the fixture recorded with the unmodified reference (tests/golden/make_golden.py, reference_boundary);
+what we return and write is checked against what the reference's stage code and readers (CouplingsModel
+model.py:317-400, read_raw_ec_file pairs.py:34-65, parse_plmc_log tools.py:20-108) made of it.  The numerical
+engine injected here is the test-only oracle engine; the same host code runs over the CUDA engine in
+tests/test_gpu_reference_protocol.py.
 """
-import functools
+import gzip
 import os
+import subprocess
+import sys
 
 import numpy as np
 import pytest
 
-import ref_harness
-
-pytestmark = pytest.mark.skipif(not ref_harness.available(), reason="reference not present (/root/reference or baseline/_ref)")
+import reference_golden as rg
 
 
 @pytest.fixture(scope="module")
 def ref():
-    ref_harness.install()
-    import evcouplings.couplings.tools as ct
-    import evcouplings.couplings.protocol as cpr
-    import evcouplings.couplings.model as cm
-    import evcouplings.couplings.pairs as cp
-    return dict(ct=ct, cpr=cpr, cm=cm, cp=cp)
-
-
-def _kwargs(prefix, a2m, L, ignore_gaps):
-    return dict(
-        protocol="standard", prefix=prefix, alignment_file=a2m, focus_mode=True, focus_sequence="seq0/1-%d" % L,
-        theta=0.8, alphabet=None, segments=[["A_1", "aa", "seq0", 1, L, list(range(1, L + 1))]],
-        ignore_gaps=ignore_gaps, iterations=30, lambda_h=0.01, lambda_J=0.01, lambda_J_times_Lq=True,
-        lambda_group=None, scale_clusters=None, cpu=2, plmc="plmc", reuse_ecs=False, min_sequence_distance=6,
-        frequencies_file=None, scoring_model="skewnormal",
-    )
+    return rg.load()
 
 
 @pytest.mark.parametrize("ignore_gaps", [True, False])
@@ -43,116 +29,114 @@ def test_reference_standard_protocol_over_our_run_plmc(ref, tmp_path, ignore_gap
     from evcouplings_b200 import synthetic, tools
     from cpu_engine import OracleEngine
     from oracle import plm_oracle as po
+    meta, arr = ref
+    name = "standard_it30_ig%d" % int(ignore_gaps)
+    rec = meta[name]
     N, L = 200, 40                      # BASELINE configs[0]
     codes = synthetic.synthetic_msa_codes(N, L, 1)
-    a2m = str(tmp_path / "cfg1.a2m")
-    synthetic.write_a2m(a2m, codes)
-    captured = {}
+    synthetic.write_a2m(str(tmp_path / "cfg1.a2m"), codes)
+    args = [rg.subst(a, tmp_path) for a in rec["args"]]
+    kwargs = {k: rg.subst(v, tmp_path) for k, v in rec["kwargs"].items()}
 
-    def run_plmc(*args, **kwargs):
-        res, run = tools.run_plmc(*args, engine=OracleEngine(), return_run=True, **kwargs)
-        captured["run"], captured["kwargs"], captured["args"] = run, kwargs, args
-        return res
-
-    ct = ref["ct"]
-    original = ct.run_plmc
-    ct.run_plmc = run_plmc
-    try:
-        prefix = str(tmp_path / "out" / "job")
-        outcfg = ref["cpr"].run(**_kwargs(prefix, a2m, L, ignore_gaps))
-    finally:
-        ct.run_plmc = original
-
-    # the protocol handed us lambda_J already scaled by (q_eff - 1) * (L - 1)   (protocol.py:157-179)
+    # the protocol hands us lambda_J already scaled by (q_eff - 1) * (L - 1)   (protocol.py:157-179)
     q_eff = 20 if ignore_gaps else 21
-    assert abs(captured["kwargs"]["lambda_J"] - 0.01 * (q_eff - 1) * (L - 1)) < 1e-12
-    assert captured["kwargs"]["focus_seq"] == "seq0/1-40" and captured["kwargs"]["theta"] == 0.8
+    assert abs(kwargs["lambda_J"] - 0.01 * (q_eff - 1) * (L - 1)) < 1e-12
+    assert kwargs["focus_seq"] == "seq0/1-40" and kwargs["theta"] == 0.8 and kwargs["iterations"] == 30
+    res, run = tools.run_plmc(*args, engine=OracleEngine(), return_run=True, **kwargs)
 
     # stage outputs the rest of the pipeline consumes
-    for key in ("model_file", "raw_ec_file", "ec_file"):
-        assert os.path.getsize(outcfg[key]) > 0
-    assert outcfg["num_sites"] == L and outcfg["num_valid_sequences"] == N
-    assert abs(outcfg["effective_sequences"] - captured["run"].n_eff) < 0.06
-    assert outcfg["region_start"] == 1
-    assert os.path.exists(prefix + "_iteration_table.csv")
-    assert os.path.exists(prefix + ".couplings_standard_plmc.outcfg")     # restart record (YAML of PlmcResult)
+    rg.check_result_as_protocol_reads_it(meta, rec, res, run)
+    assert rec["outcfg"]["num_sites"] == L and rec["outcfg"]["num_valid_sequences"] == N
+    res.iteration_table.to_csv(str(tmp_path / "job_iteration_table.csv"))
 
     # the reference's own readers on our files
-    model = ref["cm"].CouplingsModel(outcfg["model_file"])
-    run = captured["run"]
-    assert model.L == L and model.num_symbols == q_eff and model.N_valid == N
-    assert "".join(model.alphabet) == ("ACDEFGHIKLMNPQRSTVWY" if ignore_gaps else "-ACDEFGHIKLMNPQRSTVWY")
-    h = run.x[:L * q_eff].reshape(L, q_eff)
-    assert np.allclose(model.h_i, h, atol=0, rtol=0)
-    iu, ju = np.triu_indices(L, 1)
-    J = run.x[L * q_eff:].reshape(-1, q_eff, q_eff)
-    assert np.array_equal(model.J_ij[iu, ju], J.astype(np.float64))
-    assert np.array_equal(model.J_ij[ju, iu], J.transpose(0, 2, 1).astype(np.float64))
-    assert abs(model.theta - 0.2) < 1e-7 and abs(model.N_eff - run.n_eff) < 1e-2
-    assert "".join(model.target_seq) == run.alignment.target_seq
-    ecs = ref["cp"].read_raw_ec_file(outcfg["raw_ec_file"], sort=False)
-    assert len(ecs) == L * (L - 1) // 2
-    assert np.abs(ecs["cn"].values - po.cn_scores(J, L)).max() < 1e-6
-    # the reference's own log parser accepts our log and agrees with ours
-    it_ref, fields_ref = ct.parse_plmc_log(run.log)
-    it_own, fields_own = tools.parse_plmc_log(run.log)
-    assert fields_ref == fields_own
-    assert list(it_ref.columns) == list(it_own.columns) and len(it_ref) == len(it_own) == 30
-    assert it_ref.equals(it_own)
+    m = rg.check_model_as_reference_reads_it(rec, res.param_file, run)
+    assert m["alphabet"] == ("ACDEFGHIKLMNPQRSTVWY" if ignore_gaps else "-ACDEFGHIKLMNPQRSTVWY")
+    assert abs(m["theta"] - 0.2) < 1e-7 and abs(m["n_eff"] - run.n_eff) < 1e-2
+    assert m["target_seq"] == run.alignment.target_seq
+    # same oracle fit as when the reference read it
+    J = m["J"].astype(np.float64)
+    assert np.abs(m["h"] - arr[name + "_h"]).max() < 1e-5
+    Jt = J.reshape(-1)
+    assert np.abs(Jt[arr[name + "_J_idx"]] - arr[name + "_J"]).max() < 1e-5
+    sums = np.array([Jt.sum(), np.abs(Jt).sum(), (Jt * Jt).sum()])
+    assert np.all(np.abs(sums - arr[name + "_J_sums"]) <= 1e-5 * np.abs(arr[name + "_J_sums"]) + 1e-6)
+    ecs = rg.check_ecs_as_reference_reads_them(arr, name, res.couplings_file, J, L)
+    assert np.abs(ecs["cn"] - po.cn_scores(J, L)).max() < 1e-6
+    assert np.abs(ecs["cn"] - arr[name + "_ecs_cn"]).max() < 1e-5
+    # the reference's own log parser on our log agrees with ours
+    it = rg.check_log_as_reference_parses_it(rec, run.log, 30)
+    fx_ref = np.array([float(r[3]) for r in rec["iter_rows"]])
+    assert np.abs(it["fx"].astype(float).values - fx_ref).max() <= 1e-5 * np.abs(fx_ref).max()
 
 
 def test_reference_parse_of_realistic_failure_modes(ref):
     """mandatory log lines: the reference raises KeyError without them (tools.py:97-99); ours too."""
     from evcouplings_b200 import tools
-    with pytest.raises(KeyError):
-        ref["ct"].parse_plmc_log("nothing useful")
+    meta, _ = ref
+    assert meta["parse_failure"] == "KeyError"
     with pytest.raises(KeyError):
         tools.parse_plmc_log("nothing useful")
 
 
-def test_product_ingest_on_real_pabp_alignment(golden_dir):
-    """product ingest on the real A2M shipped with the reference == the golden fixture (which the oracle's
-    per-character restatement produced and plmc's own header / weights confirm: 151,496 valid + 545 invalid)."""
+def test_product_ingest_on_real_pabp_alignment(golden_dir, tmp_path):
+    """product ingest on a seeded sample of the real A2M shipped with the reference (its focus record and 1,000
+    others, 100 of them invalid) == the matching rows of the golden fixture (which the oracle's per-character
+    restatement produced and plmc's own header / weights confirm: 151,496 valid + 545 invalid)."""
     from evcouplings_b200 import msa
-    path = os.path.join(ref_harness.REFERENCE_ROOT, "notebooks", "example", "PABP_YEAST.a2m")
-    if not os.path.exists(path):
-        pytest.skip("the example alignment ships only with the full reference checkout")
-    ali = msa.load_alignment(path, focus="PABP_YEAST", ignore_gaps=True)
+    path = tmp_path / "PABP_YEAST_sample.a2m"
+    with gzip.open(os.path.join(golden_dir, "pabp_sample.a2m.gz"), "rb") as f:
+        path.write_bytes(f.read())
+    rows = np.load(os.path.join(golden_dir, "pabp_sample_rows.npy"))
+    ali = msa.load_alignment(str(path), focus="PABP_YEAST", ignore_gaps=True)
     c = np.load(os.path.join(golden_dir, "pabp_codes.npz"))
-    valid = np.unpackbits(c["valid_packed"])[: int(c["n_total"])].astype(bool)
-    assert np.array_equal(ali.codes, c["codes"]) and np.array_equal(ali.valid, valid)
+    valid_all = np.unpackbits(c["valid_packed"])[: int(c["n_total"])].astype(bool)
+    valid = valid_all[rows]
+    codes = c["codes"][(np.cumsum(valid_all) - 1)[rows[valid]]]
+    assert np.array_equal(ali.valid, valid) and np.array_equal(ali.codes, codes)
     assert ali.target_seq == str(c["target_seq"]) and np.array_equal(ali.index_list, c["index_list"])
-    assert (ali.n_valid, ali.n_total - ali.n_valid, ali.region_start, ali.num_total_sites) == (151496, 545, 115, 96)
+    assert (ali.n_valid, ali.n_total - ali.n_valid, ali.region_start, ali.num_total_sites) == \
+        (int(valid.sum()), int((~valid).sum()), 115, 96)
+    assert (~valid).sum() == 100
 
 
 def test_unmodified_reference_run_plmc_over_plmc_compatible_cli(ref, tmp_path):
-    """Secondary plug point: the reference's OWN run_plmc (tools.py:126-307: argv, subprocess, stderr parsing,
-    output checks) drives our plmc-compatible executable.  The wrapper used here injects the test-only oracle
-    engine (no GPU in this container); bin/evcplm-plmc is the same entry point with the CUDA engine."""
+    """Secondary plug point: the argv the reference's OWN run_plmc (tools.py:126-307) builds drives our
+    plmc-compatible executable; its stderr, parsed as the reference parses it, gives the reference's recorded
+    PlmcResult.  The wrapper used here injects the test-only oracle engine; bin/evcplm-plmc is the same
+    entry point with the CUDA engine."""
     import stat
-    import sys as _sys
-    from evcouplings_b200 import synthetic
+    from evcouplings_b200 import synthetic, tools
     from oracle import plm_oracle as po
+    meta, _ = ref
+    rec = meta["cli_cpu"]
     codes = synthetic.synthetic_msa_codes(150, 16, 3)
-    a2m = str(tmp_path / "in.a2m")
-    synthetic.write_a2m(a2m, codes)
+    synthetic.write_a2m(str(tmp_path / "in.a2m"), codes)
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     wrapper = tmp_path / "plmc_test_wrapper"
     wrapper.write_text(
         "#!%s\nimport sys\nsys.path.insert(0, %r); sys.path.insert(0, %r)\n"
         "from cpu_engine import OracleEngine\nfrom evcouplings_b200.plmc_cli import main\n"
-        "sys.exit(main(engine=OracleEngine()))\n" % (_sys.executable, root, os.path.join(root, "tests")))
+        "sys.exit(main(engine=OracleEngine()))\n" % (sys.executable, root, os.path.join(root, "tests")))
     wrapper.chmod(wrapper.stat().st_mode | stat.S_IEXEC)
-    ecs, model = str(tmp_path / "o" / "x_ECs.txt"), str(tmp_path / "o" / "x.model")
-    res = ref["ct"].run_plmc(a2m, ecs, model, focus_seq="seq0/1-16", alphabet=None, theta=0.8, scale=None,
-                             ignore_gaps=True, iterations=12, lambda_h=0.01, lambda_J=2.5, lambda_g=None, cpu=2,
-                             binary=str(wrapper))
-    assert res.num_valid_seqs == 150 and res.num_total_seqs == 150 and res.num_valid_sites == 16
-    assert res.focus_seq_index == 1 and res.region_start == 1
-    assert res.optimization_status == "LBFGSERR_MAXIMUMITERATION" and len(res.iteration_table) == 12
+    argv = [rg.subst(a, tmp_path) for a in rec["argv"]]
+    p = subprocess.run([str(wrapper)] + argv, capture_output=True, text=True)
+    assert p.returncode == 0, p.stderr
+    it, fields = tools.parse_plmc_log(p.stderr)
+    want = rec["result"]
+    ecs, model = rg.subst(want["couplings_file"], tmp_path), rg.subst(want["param_file"], tmp_path)
+    assert os.path.getsize(ecs) > 0 and os.path.getsize(model) > 0
+    got = dict(zip(["focus_seq_index", "num_valid_seqs", "num_total_seqs", "num_valid_sites", "num_total_sites",
+                    "region_start", "effective_samples", "optimization_status"], fields))
+    assert abs(got.pop("effective_samples") - want["effective_samples"]) < 0.06
+    assert got == {k: v for k, v in want.items() if k in got}
+    assert got["num_valid_seqs"] == 150 and got["num_total_seqs"] == 150 and got["num_valid_sites"] == 16
+    assert got["focus_seq_index"] == 1 and got["region_start"] == 1
+    assert got["optimization_status"] == "LBFGSERR_MAXIMUMITERATION"
+    assert list(it.columns) == rec["iter_columns"] and len(it) == rec["iter_len"] == 12
     m = po.read_model(model)
     assert (m["L"], m["q"], m["num_iter"]) == (16, 20, 12) and abs(m["theta"] - 0.2) < 1e-6
-    assert abs(m["lambda_J"] - 2.5) < 1e-6 and abs(res.effective_samples - m["n_eff"]) < 0.06
+    assert abs(m["lambda_J"] - 2.5) < 1e-6 and abs(fields[6] - m["n_eff"]) < 0.06
     assert len(open(ecs).read().strip().split("\n")) == 16 * 15 // 2
 
 
@@ -171,34 +155,28 @@ def test_plmc_cli_argument_handling():
 
 
 def test_reference_complex_protocol_over_our_run_plmc(ref, tmp_path):
-    """BASELINE configs[4] flavour (EVcomplex concatenated two-chain alignment): the reference's ``complex``
-    protocol (protocol.py:480-594; same infer_plmc -> run_plmc boundary, two segments, inter-chain EC table)
-    runs unmodified over our run_plmc.  Small shapes here (2 x 12 sites); the engine itself is parity- and
-    bench-tested at L=800 on the GPU."""
-    import pandas as pd
+    """BASELINE configs[4] flavour (EVcomplex concatenated two-chain alignment): the call the reference's
+    ``complex`` protocol (protocol.py:480-594; same infer_plmc -> run_plmc boundary, two segments, inter-chain
+    EC table) makes is replayed over our run_plmc.  Small shapes here (2 x 12 sites); the engine itself is
+    parity- and bench-tested at L=800 on the GPU."""
     from evcouplings_b200 import synthetic, tools
     from cpu_engine import OracleEngine
+    meta, arr = ref
+    rec = meta["complex"]
     N, L1, L2 = 160, 12, 12
     L = L1 + L2
     codes = synthetic.synthetic_msa_codes(N, L, 8)
-    a2m = str(tmp_path / "complex.a2m")
-    synthetic.write_a2m(a2m, codes, focus_name="A_B")          # header "A_B/1-24" like complex/alignment.py:85-92
-    ct = ref["ct"]
-    original = ct.run_plmc
-    ct.run_plmc = lambda *a, **k: tools.run_plmc(*a, engine=OracleEngine(), **k)
-    try:
-        prefix = str(tmp_path / "cx" / "job")
-        kw = _kwargs(prefix, a2m, L, True)
-        kw.update(protocol="complex", focus_sequence="A_B/1-%d" % L, use_all_ecs_for_scoring=False,
-                  segments=[["A_1", "aa", "A", 1, L1, list(range(1, L1 + 1))],
-                            ["B_1", "aa", "B", 1, L2, list(range(1, L2 + 1))]])
-        outcfg = ref["cpr"].run(**kw)
-    finally:
-        ct.run_plmc = original
-    assert outcfg["num_sites"] == L and outcfg["num_valid_sequences"] == N
-    inter = pd.read_csv(outcfg["inter_ec_file"])
-    assert len(inter) == L1 * L2 and set(inter["segment_i"]) == {"A_1"} and set(inter["segment_j"]) == {"B_1"}
-    allecs = pd.read_csv(outcfg["ec_file"])
-    assert {"i", "j", "segment_i", "segment_j", "cn", "probability"} <= set(allecs.columns)
-    model = ref["cm"].CouplingsModel(outcfg["model_file"])
-    assert model.L == L and model.num_symbols == 20
+    synthetic.write_a2m(str(tmp_path / "complex.a2m"), codes, focus_name="A_B")   # "A_B/1-24" like complex/alignment.py:85-92
+    args = [rg.subst(a, tmp_path) for a in rec["args"]]
+    kwargs = {k: rg.subst(v, tmp_path) for k, v in rec["kwargs"].items()}
+    assert kwargs["focus_seq"] == "A_B/1-%d" % L
+    res, run = tools.run_plmc(*args, engine=OracleEngine(), return_run=True, **kwargs)
+    rg.check_result_as_protocol_reads_it(meta, rec, res, run)
+    assert rec["outcfg"]["num_sites"] == L and rec["outcfg"]["num_valid_sequences"] == N
+    m = rg.check_model_as_reference_reads_it(rec, res.param_file, run)
+    assert m["L"] == L and m["q"] == 20
+    ecs = rg.check_ecs_as_reference_reads_them(arr, "complex", res.couplings_file, m["J"], L)
+    # the reference's inter-chain table: the raw ECs with i in segment A_1 and j in segment B_1
+    inter = int(((ecs["i"] <= L1) & (ecs["j"] > L1)).sum())
+    assert inter == rec["inter_ecs"]["rows"] == L1 * L2
+    assert rec["inter_ecs"]["segment_i"] == ["A_1"] and rec["inter_ecs"]["segment_j"] == ["B_1"]
