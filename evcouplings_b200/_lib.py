@@ -12,6 +12,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "csrc", "libevcplm.so")
 ABI_VERSION = 2
+EVC_NOT_SPD = 2      # evc_spd_inverse_f64: the matrix is not positive definite
 
 
 class EngineUnavailableError(RuntimeError):
@@ -98,6 +99,14 @@ PROTOTYPES = {
     "evc_ec_scores": (ctypes.c_int, [c_void_p, c_void_p, c_void_p, c_i32, c_i32, c_void_p, c_void_p, c_void_p, c_void_p]),
     "evc_plm_energies": (ctypes.c_int, [c_void_p, c_void_p, c_void_p, c_void_p]),
     "evc_fn_scores": (ctypes.c_int, [c_void_p, c_i32, c_i32, c_void_p, c_void_p]),
+    "evc_mf_weighted_counts_f64": (ctypes.c_int, [c_void_p, c_void_p, c_i64, c_i32, c_i32, c_f64, c_void_p, c_void_p]),
+    "evc_mf_covariance": (ctypes.c_int, [c_void_p, c_i32, c_i32, c_f64, c_void_p, c_void_p, c_void_p, c_void_p,
+                                         c_void_p]),
+    "evc_spd_inverse_f64": (ctypes.c_int, [c_void_p, c_i64, c_void_p, c_void_p, c_void_p]),
+    "evc_mf_couplings_fields": (ctypes.c_int, [c_void_p, c_void_p, c_i32, c_i32, c_void_p, c_void_p, c_void_p]),
+    "evc_mf_di_scores": (ctypes.c_int, [c_void_p, c_void_p, c_i32, c_i32, c_void_p, c_void_p, c_void_p]),
+    "evc_ec_scores_f64": (ctypes.c_int, [c_void_p, c_void_p, c_void_p, c_i32, c_i32, c_void_p, c_void_p, c_void_p,
+                                         c_void_p]),
 }
 
 _lib = None

@@ -549,4 +549,78 @@ int evc_fn_scores(const float *d_J_tri, int32_t L, int32_t q, float *d_fn, void 
     return fn_scores(d_J_tri, L, q, d_fn, as_stream(stream));
 }
 
+// ---- mean-field DCA (mean_field.cu) ----------------------------------------------------------------------
+static int mf_check_dims(const char *what, int32_t L, int32_t q)
+{
+    if (L < 2 || q < 2 || q > 21) {
+        set_error(std::string(what) + ": need L >= 2 and 2 <= q <= 21");
+        return 1;
+    }
+    return 0;
+}
+
+int evc_mf_weighted_counts_f64(const uint8_t *d_codes, const double *d_weights, int64_t N, int32_t L, int32_t q,
+                               double n_eff, double *d_F, void *stream)
+{
+    if (!d_codes || !d_weights || !d_F || N < 1) { set_error("evc_mf_weighted_counts_f64: bad argument"); return 1; }
+    if (mf_check_dims("evc_mf_weighted_counts_f64", L, q)) return 1;
+    if (!(n_eff > 0.0)) { set_error("evc_mf_weighted_counts_f64: n_eff must be > 0"); return 1; }
+    return mf_weighted_counts(d_codes, d_weights, N, L, q, n_eff, d_F, as_stream(stream));
+}
+
+int evc_mf_covariance(const double *d_F, int32_t L, int32_t q, double pseudo_count, double *d_C, double *d_fi,
+                      double *d_rfi, double *d_fij_tri, void *stream)
+{
+    if (!d_F) { set_error("evc_mf_covariance: null pointer"); return 1; }
+    if (mf_check_dims("evc_mf_covariance", L, q)) return 1;
+    return mf_covariance(d_F, L, q, pseudo_count, d_C, d_fi, d_rfi, d_fij_tri, as_stream(stream));
+}
+
+int evc_spd_inverse_f64(double *d_A, int64_t n, double *d_work, int32_t *info_out, void *stream)
+{
+    if (!d_A || !d_work || !info_out || n < 1) { set_error("evc_spd_inverse_f64: bad argument"); return 1; }
+    *info_out = 0;
+    cudaStream_t st = as_stream(stream);
+    int *d_info = nullptr;
+    EVC_CUDA(cudaMallocAsync(&d_info, sizeof(int), st));
+    const int rc = spd_inverse(d_A, n, d_work, d_info, st);
+    int info = 0;
+    if (rc == 0) {
+        EVC_CUDA(cudaMemcpyAsync(&info, d_info, sizeof(int), cudaMemcpyDeviceToHost, st));
+    }
+    EVC_CUDA(cudaFreeAsync(d_info, st));
+    EVC_CUDA(cudaStreamSynchronize(st));
+    if (rc) return rc;
+    *info_out = info;
+    if (info) {
+        set_error("evc_spd_inverse_f64: matrix is not positive definite (non-positive pivot at column " +
+                  std::to_string(info) + ")");
+        return EVC_NOT_SPD;
+    }
+    return 0;
+}
+
+int evc_mf_couplings_fields(const double *d_Cinv, const double *d_rfi, int32_t L, int32_t q, double *d_J_tri,
+                            double *d_h, void *stream)
+{
+    if (!d_Cinv || !d_rfi) { set_error("evc_mf_couplings_fields: null pointer"); return 1; }
+    if (mf_check_dims("evc_mf_couplings_fields", L, q)) return 1;
+    return mf_couplings_fields(d_Cinv, d_rfi, L, q, d_J_tri, d_h, as_stream(stream));
+}
+
+int evc_mf_di_scores(const double *d_J_tri, const double *d_rfi, int32_t L, int32_t q, double *d_di,
+                     int32_t *d_iters, void *stream)
+{
+    if (!d_J_tri || !d_rfi || !d_di) { set_error("evc_mf_di_scores: null pointer"); return 1; }
+    if (mf_check_dims("evc_mf_di_scores", L, q)) return 1;
+    return mf_di_scores(d_J_tri, d_rfi, L, q, d_di, d_iters, as_stream(stream));
+}
+
+int evc_ec_scores_f64(const double *d_J_tri, const double *d_fij_tri, const double *d_fi, int32_t L, int32_t q,
+                      double *d_fn_raw, double *d_fn_zero_sum, double *d_mi, void *stream)
+{
+    if (!d_J_tri) { set_error("evc_ec_scores_f64: null pointer"); return 1; }
+    return ec_scores_f64(d_J_tri, d_fij_tri, d_fi, L, q, d_fn_raw, d_fn_zero_sum, d_mi, as_stream(stream));
+}
+
 }  // extern "C"

@@ -117,6 +117,19 @@ int ec_scores(const float *d_J, const float *d_fij, const float *d_fi, int L, in
               float *d_fn_zs, float *d_mi, cudaStream_t st);
 int plm_energies(const PlmGeom &g, const float *d_W, const float *d_x, const uint32_t *d_msa4, float *d_epart,
                  double *d_out, cudaStream_t st);
+int ec_scores_f64(const double *d_J, const double *d_fij, const double *d_fi, int L, int q, double *d_fn_raw,
+                  double *d_fn_zs, double *d_mi, cudaStream_t st);
+
+// mean_field.cu (mean-field DCA, fp64)
+int mf_weighted_counts(const uint8_t *d_codes, const double *d_w, int64_t N, int L, int q, double n_eff, double *d_F,
+                       cudaStream_t st);
+int mf_covariance(const double *d_F, int L, int q, double pc, double *d_C, double *d_fi, double *d_rfi,
+                  double *d_fij_tri, cudaStream_t st);
+int spd_inverse(double *d_A, int64_t n, double *d_X, int *d_info, cudaStream_t st);
+int mf_couplings_fields(const double *d_Cinv, const double *d_rfi, int L, int q, double *d_J_tri, double *d_h,
+                        cudaStream_t st);
+int mf_di_scores(const double *d_J_tri, const double *d_rfi, int L, int q, double *d_di, int *d_iters,
+                 cudaStream_t st);
 
 // vecops.cu
 int vec_dot(const float *a, const float *b, int64_t n, double *out, cudaStream_t st);

@@ -13,16 +13,18 @@
 
 namespace evc {
 
-__global__ void ec_block_scores_kernel(const float *__restrict__ J, const float *__restrict__ fij,
-                                       const float *__restrict__ fi, int L, int q, int64_t npairs,
-                                       float *__restrict__ fn_raw, float *__restrict__ fn_zs,
-                                       float *__restrict__ mi)
+// Real = float for the PLM models; Real = double for the mean-field scores (accumulation is fp64 in both)
+template <typename Real>
+__global__ void ec_block_scores_kernel(const Real *__restrict__ J, const Real *__restrict__ fij,
+                                       const Real *__restrict__ fi, int L, int q, int64_t npairs,
+                                       Real *__restrict__ fn_raw, Real *__restrict__ fn_zs,
+                                       Real *__restrict__ mi)
 {
     const int64_t p = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     const int lane = threadIdx.x & 31;
     if (p >= npairs) return;
     const int qq = q * q;
-    const float *B = J + p * qq;
+    const Real *B = J + p * qq;
     // lane a (< q) owns row a: row sum, sum of squares; column sums via a second pass
     double rs = 0.0, ss = 0.0, cs = 0.0;
     if (lane < q) {
@@ -38,9 +40,9 @@ __global__ void ec_block_scores_kernel(const float *__restrict__ J, const float 
     const double R2 = warp_sum(rs * rs);
     const double C2 = warp_sum(cs * cs);
     if (lane == 0) {
-        if (fn_raw) fn_raw[p] = (float)sqrt(SS);
+        if (fn_raw) fn_raw[p] = (Real)sqrt(SS);
         double z = SS - R2 / q - C2 / q + T * T / ((double)q * q);
-        if (fn_zs) fn_zs[p] = (float)sqrt(z > 0.0 ? z : 0.0);
+        if (fn_zs) fn_zs[p] = (Real)sqrt(z > 0.0 ? z : 0.0);
     }
     if (mi != nullptr && fij != nullptr) {
         // pair index -> (i, j)
@@ -48,7 +50,7 @@ __global__ void ec_block_scores_kernel(const float *__restrict__ J, const float 
         int64_t rem = p;
         while (rem >= L - 1 - i) { rem -= L - 1 - i; i++; }
         const int j = i + 1 + (int)rem;
-        const float *F = fij + p * qq;
+        const Real *F = fij + p * qq;
         double acc = 0.0;
         for (int e = lane; e < qq; e += 32) {
             const int a = e / q, b = e - a * q;
@@ -57,20 +59,33 @@ __global__ void ec_block_scores_kernel(const float *__restrict__ J, const float 
             if (pv > 0.0 && m > 0.0) acc += pv * log(pv / m);
         }
         acc = warp_sum(acc);
-        if (lane == 0) mi[p] = (float)acc;
+        if (lane == 0) mi[p] = (Real)acc;
     }
+}
+
+template <typename Real>
+static int ec_scores_t(const Real *d_J, const Real *d_fij, const Real *d_fi, int L, int q, Real *d_fn_raw,
+                       Real *d_fn_zs, Real *d_mi, cudaStream_t st)
+{
+    const int64_t npairs = (int64_t)L * (L - 1) / 2;
+    if (npairs == 0) return 0;
+    if (q > 32) { set_error("ec_scores: q > 32 not supported"); return 1; }
+    ec_block_scores_kernel<Real><<<(unsigned)ceil_div(npairs, 8), 256, 0, st>>>(d_J, d_fij, d_fi, L, q, npairs,
+                                                                              d_fn_raw, d_fn_zs, d_mi);
+    EVC_KERNEL_CHECK();
+    return 0;
 }
 
 int ec_scores(const float *d_J, const float *d_fij, const float *d_fi, int L, int q, float *d_fn_raw,
               float *d_fn_zs, float *d_mi, cudaStream_t st)
 {
-    const int64_t npairs = (int64_t)L * (L - 1) / 2;
-    if (npairs == 0) return 0;
-    if (q > 32) { set_error("ec_scores: q > 32 not supported"); return 1; }
-    ec_block_scores_kernel<<<(unsigned)ceil_div(npairs, 8), 256, 0, st>>>(d_J, d_fij, d_fi, L, q, npairs, d_fn_raw,
-                                                                        d_fn_zs, d_mi);
-    EVC_KERNEL_CHECK();
-    return 0;
+    return ec_scores_t(d_J, d_fij, d_fi, L, q, d_fn_raw, d_fn_zs, d_mi, st);
+}
+
+int ec_scores_f64(const double *d_J, const double *d_fij, const double *d_fi, int L, int q, double *d_fn_raw,
+                  double *d_fn_zs, double *d_mi, cudaStream_t st)
+{
+    return ec_scores_t(d_J, d_fij, d_fi, L, q, d_fn_raw, d_fn_zs, d_mi, st);
 }
 
 // ---- f2: energies --------------------------------------------------------------------------------

@@ -104,6 +104,69 @@ class CudaEngine(object):
         self.all_reduce(d_counts)
         return d_counts
 
+    # -- mean-field DCA (fp64, csrc/mean_field.cu) ------------------------------------------------
+    def mean_field(self, codes, weights, q, pseudo_count, timings=None):
+        """Mean-field DCA of (N, L) codes (alphabet order, last state = reference state) with fp64 sequence
+        weights, on device-resident buffers.  Returns float64 numpy arrays: fi, rfi (L, q), h (L, q), fij_tri and
+        J_tri (pairs i<j, q, q), di, fn (zero-sum gauge), mi (pairs i<j) and di_iters.  ``timings``: a dict that
+        receives the milliseconds of each stage (CUDA events on the engine's stream)."""
+        torch = _torch()
+        lib, vp = self.lib, self.ptr
+        codes = np.ascontiguousarray(codes, dtype=np.uint8)
+        N, L = codes.shape
+        n, Lq, npairs = L * (q - 1), L * q, L * (L - 1) // 2
+        weights = np.ascontiguousarray(weights, dtype=np.float64)
+        n_eff = float(weights.sum())
+        dev, f64, st = self.device, torch.float64, self.stream()
+        events = []
+
+        def mark(name):
+            if timings is not None:
+                ev = torch.cuda.Event(enable_timing=True)
+                ev.record(torch.cuda.current_stream(dev))
+                events.append((name, ev))
+
+        d_codes = torch.from_numpy(codes).to(dev)
+        d_w = torch.from_numpy(weights).to(dev)
+        mark("start")
+        F = torch.empty((Lq, Lq), dtype=f64, device=dev)
+        _lib.check(lib.evc_mf_weighted_counts_f64(vp(d_codes), vp(d_w), N, L, q, n_eff, vp(F), st),
+                   "evc_mf_weighted_counts_f64")
+        mark("counts")
+        C = torch.empty((n, n), dtype=f64, device=dev)
+        fi = torch.empty((L, q), dtype=f64, device=dev)
+        rfi = torch.empty((L, q), dtype=f64, device=dev)
+        fij = torch.empty((npairs, q, q), dtype=f64, device=dev)
+        _lib.check(lib.evc_mf_covariance(vp(F), L, q, float(pseudo_count), vp(C), vp(fi), vp(rfi), vp(fij), st),
+                   "evc_mf_covariance")
+        mark("covariance")
+        del F
+        work = torch.empty((n, n), dtype=f64, device=dev)
+        info = ctypes.c_int32(0)
+        _lib.check(lib.evc_spd_inverse_f64(vp(C), n, vp(work), ctypes.byref(info), st), "evc_spd_inverse_f64")
+        mark("inverse")
+        del work
+        J = torch.empty((npairs, q, q), dtype=f64, device=dev)
+        h = torch.empty((L, q), dtype=f64, device=dev)
+        _lib.check(lib.evc_mf_couplings_fields(vp(C), vp(rfi), L, q, vp(J), vp(h), st), "evc_mf_couplings_fields")
+        mark("fields")
+        del C
+        di = torch.empty(npairs, dtype=f64, device=dev)
+        iters = torch.empty(npairs, dtype=torch.int32, device=dev)
+        _lib.check(lib.evc_mf_di_scores(vp(J), vp(rfi), L, q, vp(di), vp(iters), st), "evc_mf_di_scores")
+        mark("di")
+        scores = torch.empty((2, npairs), dtype=f64, device=dev)
+        _lib.check(lib.evc_ec_scores_f64(vp(J), vp(fij), vp(fi), L, q, None, vp(scores[0]), vp(scores[1]), st),
+                   "evc_ec_scores_f64")
+        mark("scores")
+        torch.cuda.synchronize(dev)
+        if timings is not None:
+            for (_, a), (name, b) in zip(events, events[1:]):
+                timings[name] = a.elapsed_time(b)
+        s = scores.cpu().numpy()
+        return dict(fi=fi.cpu().numpy(), rfi=rfi.cpu().numpy(), h=h.cpu().numpy(), fij_tri=fij.cpu().numpy(),
+                    J_tri=J.cpu().numpy(), di=di.cpu().numpy(), fn=s[0], mi=s[1], di_iters=iters.cpu().numpy())
+
     # -- (a) PLM ---------------------------------------------------------------------------
     def plm_problem(self, codes, weights, q, gap_code, lambda_h, lambda_J, m=6, backward=None, forward=None,
                     precision=None):

@@ -44,23 +44,42 @@ def write_model_file(path, L, q, n_valid, n_invalid, num_iter, theta_plmc, lambd
     int32[5] L q N_valid N_invalid num_iter | float32[5] theta lambda_h lambda_J lambda_group N_eff |
     char[q] alphabet | float32[N] weights | char[L] target_seq | int32[L] index_list |
     float32[L][q] f_i | float32[L][q] h_i | float32[npairs][q][q] f_ij | float32[npairs][q][q] J_ij"""
+    if lambda_h < 0:
+        raise ValueError("lambda_h < 0 marks a mean-field model in this format; refusing to write it")
+    _write_plmc_v2(path, L, q, n_valid, n_invalid, num_iter, theta_plmc, lambda_h, lambda_J, lambda_group, n_eff,
+                   alphabet, weights_all, target_seq, index_list, fi, h, fij_tri, J_tri, "<f4")
+
+
+def write_mean_field_model_file(path, L, q, n_valid, theta, pseudo_count, n_eff, alphabet, weights, target_seq,
+                                index_list, fi, h, fij_tri, J_tri, precision="float32"):
+    """A mean-field model in the plmc_v2 layout, as the reference's MeanFieldCouplingsModel.to_file writes it:
+    lambda_h = -pseudo_count (the reference's reader takes lambda_h < 0 as "mean-field model"), lambda_J,
+    lambda_group and num_iter = -1, N_invalid = 0 with the weights of the valid sequences only; the real-valued
+    fields in ``precision`` (float16 / float32 / float64)."""
+    dtype = np.dtype(precision).newbyteorder("<")
+    if dtype.kind != "f":
+        raise ValueError("precision must be a floating-point type")
+    _write_plmc_v2(path, L, q, n_valid, 0, -1, theta, -pseudo_count, -1, -1, n_eff, alphabet, weights, target_seq,
+                   index_list, fi, h, fij_tri, J_tri, dtype)
+
+
+def _write_plmc_v2(path, L, q, n_valid, n_invalid, num_iter, theta, lambda_h, lambda_J, lambda_group, n_eff,
+                   alphabet, weights_all, target_seq, index_list, fi, h, fij_tri, J_tri, dtype):
     alphabet = str(alphabet)
     target_seq = str(target_seq)
     npairs = L * (L - 1) // 2
-    fi = np.asarray(fi, dtype="<f4").reshape(L, q)
-    h = np.asarray(h, dtype="<f4").reshape(L, q)
-    fij_tri = np.asarray(fij_tri, dtype="<f4").reshape(npairs, q, q)
-    J_tri = np.asarray(J_tri, dtype="<f4").reshape(npairs, q, q)
-    weights_all = np.asarray(weights_all, dtype="<f4")
+    fi = np.asarray(fi, dtype=dtype).reshape(L, q)
+    h = np.asarray(h, dtype=dtype).reshape(L, q)
+    fij_tri = np.asarray(fij_tri, dtype=dtype).reshape(npairs, q, q)
+    J_tri = np.asarray(J_tri, dtype=dtype).reshape(npairs, q, q)
+    weights_all = np.asarray(weights_all, dtype=dtype)
     if len(alphabet) != q or len(target_seq) != L or len(index_list) != L:
         raise ValueError("inconsistent model dimensions")
     if weights_all.shape != (n_valid + n_invalid,):
         raise ValueError("weights must cover valid + invalid sequences")
-    if lambda_h < 0:
-        raise ValueError("lambda_h < 0 marks a mean-field model in this format; refusing to write it")
     with open(path, "wb") as f:
         np.array([L, q, n_valid, n_invalid, num_iter], dtype="<i4").tofile(f)
-        np.array([theta_plmc, lambda_h, lambda_J, lambda_group, n_eff], dtype="<f4").tofile(f)
+        np.array([theta, lambda_h, lambda_J, lambda_group, n_eff], dtype=dtype).tofile(f)
         f.write(alphabet.encode("ascii"))
         weights_all.tofile(f)
         f.write(target_seq.encode("ascii"))

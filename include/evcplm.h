@@ -233,6 +233,39 @@ int evc_plm_energies(evc_plm_t *h, const float *d_x, double *d_out, void *stream
 /* ---- a10: EC scores (Frobenius norm of each J block, raw gauge) ---------- */
 int evc_fn_scores(const float *d_J_tri, int32_t L, int32_t q, float *d_fn /* L(L-1)/2 */, void *stream);
 
+/* ---- mean-field DCA (the couplings stage's `mean_field` protocol: evcouplings/couplings/mean_field.py) -------
+ * Everything in fp64.  Sites L >= 2, states q in 2..21 (the gap is a state, alphabet order, last state = the
+ * reference state of the model), n = L*(q-1).  All arrays are device arrays, row-major.
+ *   evc_mf_weighted_counts_f64: d_F ((L*q) x (L*q), symmetric) at row i*q+a, column j*q+b =
+ *       sum_s w_s [s_i = a][s_j = b] / n_eff  (so the (i,i) blocks hold f_i on their diagonal).
+ *   evc_mf_covariance: from d_F and the pseudo-count pc, any output may be NULL:
+ *       d_C (n x n): rf_ij[a][b] - rf_i[a] rf_j[b], a, b < q-1, with rf_i = (1-pc) f_i + pc/q,
+ *           rf_ij = (1-pc) f_ij + pc/q^2 for i != j and (1-pc) f_i[a] d_ab + (pc/q) d_ab for i == j;
+ *       d_fi, d_rfi (L x q): raw and regularised single-site frequencies;
+ *       d_fij_tri (L(L-1)/2 blocks of q x q, pairs i<j row-major): raw pair frequencies.
+ *   evc_spd_inverse_f64: d_A (n x n, symmetric positive definite, only the lower triangle is read) is replaced by
+ *       its inverse (both triangles); d_work holds n*n doubles.  Blocked Cholesky, triangular inverse, X^T X.
+ *       Synchronous.  Returns EVC_NOT_SPD, *info_out = 1-based column of the first non-positive pivot, when the
+ *       matrix is not positive definite (d_A is then undefined); *info_out = 0 on success.
+ *   evc_mf_couplings_fields: d_J_tri (tri blocks) = -Cinv[(i,a),(j,b)] for a, b < q-1, 0 on the last state;
+ *       d_h (L x q) = log(rf_i[a] / rf_i[q-1]) - sum_{j != i} sum_b J_ij[a][b] rf_j[b].
+ *   evc_mf_di_scores: direct information of every pair (tri order) from J and the regularised f_i: the two-site
+ *       fixed point on exp(J_ij) from 1/q until the max-abs change is <= 1e-4; d_iters (may be NULL) receives
+ *       the iteration count of each pair.
+ *   evc_ec_scores_f64: evc_ec_scores in fp64 (the mean-field couplings are scored without a float32 rounding). */
+#define EVC_NOT_SPD 2
+int evc_mf_weighted_counts_f64(const uint8_t *d_codes /* N x L */, const double *d_weights, int64_t N, int32_t L,
+                               int32_t q, double n_eff, double *d_F, void *stream);
+int evc_mf_covariance(const double *d_F, int32_t L, int32_t q, double pseudo_count, double *d_C, double *d_fi,
+                      double *d_rfi, double *d_fij_tri, void *stream);
+int evc_spd_inverse_f64(double *d_A, int64_t n, double *d_work, int32_t *info_out, void *stream);
+int evc_mf_couplings_fields(const double *d_Cinv, const double *d_rfi, int32_t L, int32_t q, double *d_J_tri,
+                            double *d_h, void *stream);
+int evc_mf_di_scores(const double *d_J_tri, const double *d_rfi, int32_t L, int32_t q, double *d_di,
+                     int32_t *d_iters, void *stream);
+int evc_ec_scores_f64(const double *d_J_tri, const double *d_fij_tri, const double *d_fi, int32_t L, int32_t q,
+                      double *d_fn_raw, double *d_fn_zero_sum, double *d_mi, void *stream);
+
 #ifdef __cplusplus
 }
 #endif
